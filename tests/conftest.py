@@ -14,16 +14,36 @@ def pytest_configure(config):
 
 @pytest.fixture(scope="session")
 def ref():
-    """The unmodified reference (libsecp256k1 + CCAN sha256) compiled by oracle/Makefile."""
+    """The unmodified reference (libsecp256k1 + CCAN sha256): its recorded answers (tests/refcalls.py)."""
     from tests import util
-    return util.load_ref()
+    return util.recorded_ref()
 
 
 @pytest.fixture(scope="session")
 def cln():
-    """CLN's own plumbing (bitcoin/signature.c, common/node_id.c, gossipd/sigcheck.c), unmodified."""
+    """CLN's own plumbing (bitcoin/signature.c, common/node_id.c, gossipd/sigcheck.c), unmodified: its recorded answers."""
     from tests import util
-    return util.load_cln()
+    return util.recorded_cln()
+
+
+def _live(load):
+    try:
+        return load()
+    except RuntimeError as e:
+        pytest.skip(str(e))
+
+
+@pytest.fixture(scope="session")
+def ref_live():
+    """The reference library itself, for tests that hand the engine objects it built; skips where oracle/_ref is absent."""
+    from tests import util
+    return _live(util.load_ref)
+
+
+@pytest.fixture(scope="session")
+def cln_live():
+    from tests import util
+    return _live(util.load_cln)
 
 
 @pytest.fixture(scope="session")

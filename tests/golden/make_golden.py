@@ -24,6 +24,8 @@ exists; the GPU box only sees the generated files).  Vectors are data, not code:
   bolt3_htlc_txs.json     BOLT #3 Appendix C "commitment tx with all five HTLCs untrimmed (minimum feerate)": the five fully
                           signed HTLC transactions embedded in channeld/test/run-full_channel.c:635-673 (hex), parsed into
                           the fields BIP143 commits to, with both the remote and the local HTLC signature of each
+  bip143_libwally.json    libwally's BIP143 sighash (CLN's bitcoin_tx_hash_for_sig, oracle/_ref) of 120 seeded random
+                          transactions of 1-3 inputs and 1-6 outputs
 
 Every expected verdict written here is re-checked against oracle/_ref (the unmodified reference) at
 generation time.
@@ -402,6 +404,48 @@ def bolt3_htlc_txs():
     print("bolt3_htlc_txs:", len(out), "transactions,", sum(len(o["sigs"]) for o in out), "signatures, all valid under the reference")
 
 
+def bip143_libwally():
+    """libwally's sighash (bitcoin_tx_hash_for_sig via oracle/cln_harness.c) of the 120 seeded transactions that
+    tests/test_host_emul.py::test_bip143_bolt3_and_general_shapes_vs_libwally draws; the draws here must stay in step."""
+    cln = util.load_cln()
+    vp = ctypes.c_void_p
+    cln.cln_tx_new.restype = vp
+    cln.cln_tx_new.argtypes = [ctypes.c_uint32, ctypes.c_uint32]
+    cln.cln_tx_add_input.argtypes = [vp, ctypes.c_char_p, ctypes.c_uint32, ctypes.c_uint32]
+    cln.cln_tx_add_output.argtypes = [vp, ctypes.c_uint64, ctypes.c_char_p, ctypes.c_size_t]
+    cln.cln_tx_free.argtypes = [vp]
+    cln.cln_tx_set_input_amount.argtypes = [ctypes.c_uint64]
+    cln.cln_tal_bytes.restype = vp
+    cln.cln_tal_bytes.argtypes = [ctypes.c_char_p, ctypes.c_size_t]
+    cln.cln_tal_free.argtypes = [vp]
+    cln.cln_tx_sighash.argtypes = [vp, ctypes.c_uint, vp, ctypes.c_uint32, vp]
+    rng = np.random.default_rng(8)
+    out = []
+    for it in range(120):
+        nin, nout = int(rng.integers(1, 4)), int(rng.integers(1, 7))
+        ins = [(bytes(rng.integers(0, 256, size=32, dtype=np.uint8)), int(rng.integers(0, 9)), int(rng.integers(0, 2**32))) for _ in range(nin)]
+        outs = [(int(rng.integers(0, 2**40)), bytes(rng.integers(0, 256, size=int(rng.choice([0, 22, 34, 300])), dtype=np.uint8))) for _ in range(nout)]
+        lock = int(rng.integers(0, 2**32))
+        tx = cln.cln_tx_new(2, lock)
+        for a in ins:
+            assert cln.cln_tx_add_input(tx, *a) == 0
+        for amt, sc in outs:
+            assert cln.cln_tx_add_output(tx, amt, sc or None, len(sc)) == 0
+        inp = int(rng.integers(0, nin))
+        ws = bytes(rng.integers(0, 256, size=int(rng.choice([1, 2, 133, 252, 253, 700])), dtype=np.uint8))
+        amount = int(rng.integers(0, 2**45))
+        sht = int(rng.choice([1, 0x83, 2, 3, 0x81, 0x82]))
+        tal_ws = cln.cln_tal_bytes(ws, len(ws))
+        cln.cln_tx_set_input_amount(amount)
+        want = np.zeros(32, np.uint8)
+        cln.cln_tx_sighash(tx, inp, tal_ws, sht, P(want))
+        out.append(bytes(want).hex())
+        cln.cln_tal_free(tal_ws)
+        cln.cln_tx_free(tx)
+    json.dump(out, open(OUT + "/bip143_libwally.json", "w"), indent=0)
+    print("bip143_libwally:", len(out), "sighashes")
+
+
 if __name__ == "__main__":
     if len(sys.argv) > 1:  # regenerate only the named sets
         for name in sys.argv[1:]:
@@ -415,4 +459,5 @@ if __name__ == "__main__":
     ecmult_kat()
     ecdsa_edge_cases()
     bolt3_htlc_txs()
+    bip143_libwally()
     gossip_store_full()

@@ -90,7 +90,7 @@ def test_dropin_cln_signatures(engine, ref):
     """check_signed_hash / check_signed_hash_nodeid / check_schnorr_sig / sha256_double / pubkey_from_der with
     CLN's own argument types (opaque libsecp256k1 structs produced by the reference's parsers)."""
     lib = _dropin(engine)
-    w = util.corrupt(util.make_signed(ref, 120, seed=99), every=4)
+    w = util.corrupt(util.make_signed(120, seed=99), every=4)
     n_checked = 0
     for i in range(120):
         opk, osig = np.zeros(64, np.uint8), np.zeros(64, np.uint8)
@@ -208,7 +208,7 @@ def test_config_c1_dropin_vs_cln_own_functions(engine, ref, cln):
     check_signed_hash_nodeid / check_schnorr_sig (CLN argument types, opaque structs built by CLN's own wire
     parsers) must agree call by call with CLN's unmodified functions."""
     lib = _dropin(engine)
-    w = util.corrupt(util.make_signed(ref, 1000, seed=20260922), every=10)
+    w = util.corrupt(util.make_signed(1000, seed=20260922), every=10)
     agree = 0
     for i in range(1000):
         m, k, s, ss = (np.ascontiguousarray(w[x][i]) for x in ("msg", "pub33", "sig", "ssig"))
@@ -407,7 +407,7 @@ def test_verifier_subdaemon(ref, cln, tmp_path):
             time.sleep(0.1)
         assert os.path.exists(sock_path), "daemon did not come up"
         assert stat.S_IMODE(os.stat(sock_path).st_mode) == 0o600
-        w = util.corrupt(util.make_signed(ref, 2400, seed=21), every=6)
+        w = util.corrupt(util.make_signed(2400, seed=21), every=6)
         kinds = [(0, "pub33", "sig", 33), (1, "pubxy", "sig", 64), (2, "xonly", "ssig", 32)]
         want = [util.ref_verify(ref, k, w["msg"], w[kk], w[ss]) for k, kk, ss, _ in kinds]
         errors = []

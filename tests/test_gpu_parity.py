@@ -13,7 +13,7 @@ K33, KXY, KSCH = 0, 1, 2
 
 @pytest.fixture(scope="module")
 def workload(ref):
-    w = util.make_signed(ref, 6000, seed=20260922)
+    w = util.make_signed(6000, seed=20260922)
     return util.corrupt(w, every=7)
 
 
@@ -143,7 +143,7 @@ def test_synth_generator_is_valid_under_reference(engine, ref):
 def test_mutation_differential(engine, ref):
     """20,000 structured mutations (boundary r/s/x/m values, negated or swapped fields, random flips): GPU vs reference."""
     from tests import mutations
-    w = util.make_signed(ref, 20000, seed=321)
+    w = util.make_signed(20000, seed=321)
     cls = mutations.mutate(w, seed=10)
     for kind, (k, s) in enumerate([("pub33", "sig"), ("pubxy", "sig"), ("xonly", "ssig")]):
         want = util.ref_verify(ref, kind, w["msg"], w[k], w[s], threads=8)

@@ -35,7 +35,7 @@ def both(engine):
 
 
 def test_small_path_random_corrupted_ragged(engine, ref, both):
-    w = util.corrupt(util.make_signed(ref, 8200, seed=77), every=5)
+    w = util.corrupt(util.make_signed(8200, seed=77), every=5)
     for kind, (k, s) in enumerate(KINDS):
         want = util.ref_verify(ref, kind, w["msg"], w[k], w[s], threads=4)
         for n in (1, 2, 3, 4, 5, 31, 32, 33, 63, 64, 65, 95, 96, 97, 483, 1000, 2047, 2048, 2049, 2600, 8191, 8192, 8193, 8200):
@@ -49,7 +49,7 @@ def test_small_path_random_corrupted_ragged(engine, ref, both):
 
 
 def test_small_path_mutations_adversarial_golden(engine, ref, both):
-    w = util.make_signed(ref, 3000, seed=123)
+    w = util.make_signed(3000, seed=123)
     mutations.mutate(w, seed=9)
     for kind, (k, s) in enumerate(KINDS):
         want = util.ref_verify(ref, kind, w["msg"], w[k], w[s], threads=4)
@@ -118,7 +118,7 @@ def test_small_path_composite_entry_points(engine, ref, cln, both):
     assert np.array_equal(a, want) and np.array_equal(b, want)
     a, b = both(lambda: (engine.verify_samekey(0, pub33, hs, sig).copy(), engine.verify_samekey(1, pubxy, hs, sig).copy()))
     assert all(np.array_equal(x, want) for x in a + b)
-    w = util.corrupt(util.make_signed(ref, 90, seed=5), every=4)
+    w = util.corrupt(util.make_signed(90, seed=5), every=4)
 
     def queue():
         for i in range(90):
@@ -138,7 +138,7 @@ def test_ecdsa33_without_square_root_vs_plain_flow(engine, ref):
     default = engine.small_max()
     engine.set_small_max(0)
     try:
-        w = util.corrupt(util.make_signed(ref, 5000, seed=78), every=4)
+        w = util.corrupt(util.make_signed(5000, seed=78), every=4)
         p = 2**256 - 2**32 - 977
         for i in range(60):  # x not on the curve
             x = int.from_bytes(bytes(w["pub33"][i, 1:]), "big")
@@ -149,7 +149,7 @@ def test_ecdsa33_without_square_root_vs_plain_flow(engine, ref):
         w["pub33"][61, 1:] = 255  # x >= p
         want = util.ref_verify(ref, 0, w["msg"], w["pub33"], w["sig"], threads=4)
         assert not want[:62].any() and want.sum() > 3000
-        m = util.make_signed(ref, 3000, seed=124)
+        m = util.make_signed(3000, seed=124)
         mutations.mutate(m, seed=10)
         mwant = util.ref_verify(ref, 0, m["msg"], m["pub33"], m["sig"], threads=4)
         amsg, apub33, _, asig = adversarial.load()
@@ -159,7 +159,7 @@ def test_ecdsa33_without_square_root_vs_plain_flow(engine, ref):
         ck = np.concatenate([h(c["pub33"], 33) for c in cases])
         cs = np.concatenate([h(c["sig64"], 64) for c in cases])
         cwant = np.array([c["expected"] for c in cases], np.uint8)
-        ws = util.corrupt(util.make_signed(ref, 5000, seed=79), every=3)
+        ws = util.corrupt(util.make_signed(5000, seed=79), every=3)
         ws["xonly"][:60] = w["pub33"][:60, 1:]   # x-only keys off the curve
         ws["ssig"][60:80, 32:] = 0               # s = 0: the comb sum is the point at infinity
         swant = util.ref_verify(ref, 2, ws["msg"], ws["xonly"], ws["ssig"], threads=4)

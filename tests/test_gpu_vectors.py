@@ -109,9 +109,10 @@ def _dropin_tx(engine, cln):
     return lib
 
 
-def test_check_tx_sig_reference_signature_bolt3(engine, cln):
+def test_check_tx_sig_reference_signature_bolt3(engine, cln_live):
     """bitcoin/signature.h:120 check_tx_sig(tx, input_num, redeemscript, witness_script, key, sig) exported by the engine,
     fed the reference's own struct bitcoin_tx (libwally wally_tx inside) — BOLT #3's HTLC transactions."""
+    cln = cln_live
     C = _Cln(cln)
     lib = _dropin_tx(engine, cln)
     assert cln.cln_sizeof_bitcoin_signature() == 68
@@ -135,11 +136,12 @@ def test_check_tx_sig_reference_signature_bolt3(engine, cln):
         cln.cln_tx_free(tx)
 
 
-def test_check_tx_sig_vs_cln_own_on_arbitrary_transactions(engine, ref, cln):
+def test_check_tx_sig_vs_cln_own_on_arbitrary_transactions(engine, ref_live, cln_live):
     """Differential: the engine's check_tx_sig against CLN's OWN unmodified check_tx_sig (bitcoin/signature.c:194-221 over
     libwally's BIP143) on transactions of 1-3 inputs and 1-6 outputs (commitment-like shapes included), scripts from 1 to
     700 bytes (CLN itself asserts on an empty one: libwally refuses a non-NULL zero-length script), every sighash type incl. the ones the gate refuses, witness and non-witness script argument, SIGHASH_SINGLE
     with and without a matching output; signatures made over libwally's sighash with the signature's own type."""
+    ref, cln = ref_live, cln_live
     C = _Cln(cln)
     lib = _dropin_tx(engine, cln)
     rng = np.random.default_rng(2026)
@@ -285,7 +287,7 @@ def test_mixed_kinds_interleaved_config_c3(engine, ref):
     """BASELINE config C3 in miniature: ECDSA (33-byte and x||y keys) and BIP-340 items interleaved by a seeded shuffle
     with a kind tag per item, through sv_verify_mixed_host (device-side split per kind); every verdict vs the reference,
     at sizes on both sides of the small-path threshold; an unknown tag gives verdict 0."""
-    w = util.corrupt(util.make_signed(ref, 9000, seed=31), every=6)
+    w = util.corrupt(util.make_signed(9000, seed=31), every=6)
     rng = np.random.default_rng(6)
     for n in (1, 5, 64, 3000, 9000):
         kinds = rng.choice([0, 0, 1, 2, 2], size=n).astype(np.uint8)
@@ -366,7 +368,7 @@ def test_bip340_batch_verification_rlc(engine, ref):
     one-by-one verification), the 10 %-corrupted mix (every group falls back), encoding failures (excluded, no fallback
     needed), ragged sizes, different seeds and the system's own randomness."""
     n = 5000
-    w = util.make_signed(ref, n, seed=88)
+    w = util.make_signed(n, seed=88)
     msg, key, sig = w["msg"], w["xonly"], w["ssig"]
     v, gt, gf = engine.verify_schnorr_batch(msg, key, sig, seed32=bytes(range(32)))
     assert v.all() and gt == 5 and gf == 0
@@ -388,7 +390,7 @@ def test_bip340_batch_verification_rlc(engine, ref):
     assert np.array_equal(v, want) and list(np.nonzero(want == 0)[0]) == [100, 200, 3000, 4500, 4600]
     assert gf == 2  # groups 0 and 2; the encoding failures in group 4 needed no fallback
     # heavy damage: every group falls back, verdicts still exact
-    w3 = util.corrupt(util.make_signed(ref, 4000, seed=89), every=10)
+    w3 = util.corrupt(util.make_signed(4000, seed=89), every=10)
     want = util.ref_verify(ref, 2, w3["msg"], w3["xonly"], w3["ssig"], threads=4)
     v, gt, gf = engine.verify_schnorr_batch(w3["msg"], w3["xonly"], w3["ssig"], seed32=bytes(32))
     assert np.array_equal(v, want) and gf == gt == 4 and 0 < want.sum() < want.size

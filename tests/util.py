@@ -5,6 +5,8 @@ import subprocess
 
 import numpy as np
 
+from tests import refcalls
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 N_ORDER = 0xFFFFFFFFFFFFFFFFFFFFFFFFFFFFFFFEBAAEDCE6AF48A03BBFD25E8CD0364141
 P_FIELD = 2**256 - 2**32 - 977
@@ -12,28 +14,36 @@ _p8 = ctypes.POINTER(ctypes.c_uint8)
 
 
 def P(a):
-    return a.ctypes.data_as(_p8)
+    """A uint8 pointer to the contiguous array a; it keeps a, so that tests.refcalls can record what a call reads and writes."""
+    p = a.ctypes.data_as(_p8)
+    p._sv_arr = a
+    return p
+
+
+def _load_lib(name):
+    path = os.path.join(ROOT, "oracle", "_ref", name)
+    if not os.path.exists(path):
+        raise RuntimeError(f"oracle/_ref/{name} is missing: it is built by oracle/Makefile where the reference's sources are")
+    return ctypes.CDLL(path)
 
 
 def load_ref():
-    path = os.path.join(ROOT, "oracle", "_ref", "libsecp_ref.so")
-    if not os.path.exists(path):
-        if os.path.isdir("/root/reference"):
-            subprocess.check_call(["make", "-C", os.path.join(ROOT, "oracle"), "ref"], stdin=subprocess.DEVNULL)
-        else:
-            raise RuntimeError("oracle/_ref/libsecp_ref.so missing and /root/reference absent")
-    return ctypes.CDLL(path)
+    """The unmodified reference (libsecp256k1 + CCAN sha256), as built into oracle/_ref."""
+    return _load_lib("libsecp_ref.so")
 
 
 def load_cln():
     """CLN's own unmodified bitcoin/signature.c + gossipd/sigcheck.c over the libwally amalgamation (config C1)."""
-    path = os.path.join(ROOT, "oracle", "_ref", "libcln_ref.so")
-    if not os.path.exists(path):
-        if os.path.isdir("/root/reference"):
-            subprocess.check_call(["make", "-s", "-C", os.path.join(ROOT, "oracle"), "cln"], stdin=subprocess.DEVNULL)
-        else:
-            raise RuntimeError("oracle/_ref/libcln_ref.so missing and /root/reference absent")
-    return ctypes.CDLL(path)
+    return _load_lib("libcln_ref.so")
+
+
+def recorded_ref():
+    """load_ref()'s answers as tests/golden/refcalls.bin recorded them (see tests/refcalls.py)."""
+    return refcalls.Library("ref", load_ref)
+
+
+def recorded_cln():
+    return refcalls.Library("cln", load_cln)
 
 
 def load_port():
@@ -55,8 +65,9 @@ def ref_verify(ref, kind, msg, key, sig, threads=1):
     return out
 
 
-def make_signed(ref, n, seed):
-    """n seeded random keys/messages signed by the reference: returns dict of arrays."""
+def make_signed(n, seed):
+    """n seeded random keys/messages, signed as the reference's ref_pubkey_create / ref_ecdsa_sign / ref_schnorr_sign
+    sign them (tests/refcalls.py restates those): returns dict of arrays."""
     rng = np.random.default_rng(seed)
     sk = rng.integers(0, 256, size=(n, 32), dtype=np.uint8)
     msg = rng.integers(0, 256, size=(n, 32), dtype=np.uint8)
@@ -66,9 +77,13 @@ def make_signed(ref, n, seed):
     xonly = np.zeros((n, 32), np.uint8)
     ssig = np.zeros((n, 64), np.uint8)
     for i in range(n):
-        assert ref.ref_pubkey_create(P(sk[i]), P(pub33[i]), P(pubxy[i]))
-        assert ref.ref_ecdsa_sign(P(sk[i]), P(msg[i]), P(sig[i]))
-        assert ref.ref_schnorr_sign(P(sk[i]), P(msg[i]), P(ssig[i]), P(xonly[i]))
+        d = int.from_bytes(sk[i].tobytes(), "big")
+        m = msg[i].tobytes()
+        pubxy[i] = refcalls.base_mult(d)
+        pub33[i, 0], pub33[i, 1:] = 2 + (pubxy[i, 63] & 1), pubxy[i, :32]
+        sig[i] = np.frombuffer(refcalls.ecdsa_sign(d, m), np.uint8)
+        s, x = refcalls.schnorr_sign(d, m)
+        ssig[i], xonly[i] = np.frombuffer(s, np.uint8), np.frombuffer(x, np.uint8)
     return dict(msg=msg, pub33=pub33, pubxy=pubxy, sig=sig, xonly=xonly, ssig=ssig)
 
 

@@ -32,7 +32,7 @@ def main():
     eng = L.SigVerifier(0)
     ref = util.load_ref()
     sizes = tuple(int(x) for x in os.environ.get("SV_LATENCY_SIZES", "1,4,32,483,4096").split(","))
-    w = util.make_signed(ref, max(4096, max(sizes)), seed=7)
+    w = util.make_signed(max(4096, max(sizes)), seed=7)
     out = {"small_max": eng.small_max(), "sizes": {}, "note": "synchronous sv_verify_host calls, pageable numpy host buffers, perf_counter around the call"}
     kinds = (("ecdsa33", 0, "pub33", "sig"), ("ecdsa_xy", 1, "pubxy", "sig"), ("schnorr", 2, "xonly", "ssig"))
     for n in sizes:

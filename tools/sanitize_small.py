@@ -6,7 +6,7 @@ import lightning_b200 as L
 from tests import util
 ref = util.load_ref()
 eng = L.SigVerifier(0)
-w = util.corrupt(util.make_signed(ref, 300, seed=3), every=5)
+w = util.corrupt(util.make_signed(300, seed=3), every=5)
 for n in (1, 5, 300):
     for kind, (k, s) in enumerate([("pub33", "sig"), ("pubxy", "sig"), ("xonly", "ssig")]):
         got = eng.verify(kind, w["msg"][:n], w[k][:n], w[s][:n])
@@ -49,7 +49,7 @@ eng.set_small_max(0)  # the key search only runs above the small-batch limit
 st = eng.verify_gossip(big)
 eng.set_small_max(8192)
 print("gossip with de-duplication", int((st == 0).sum()), "of", len(big), "distinct keys", eng.last_distinct_keys())
-w2 = util.make_signed(ref, 1100, seed=4)
+w2 = util.make_signed(1100, seed=4)
 v, gt, gf = eng.verify_schnorr_batch(w2["msg"], w2["xonly"], w2["ssig"], seed32=bytes(32))
 print("schnorr batch", int(v.sum()), gt, gf)
 w2["ssig"][5, 40] ^= 1
