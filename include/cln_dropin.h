@@ -41,6 +41,8 @@ struct sha256 { union { uint32_t u32[8]; unsigned char u8[32]; } u; };  /* ccan/
 struct sha256_double { struct sha256 sha; };                           /* bitcoin/shadouble.h:9-11 */
 typedef struct { unsigned char data[64]; } secp256k1_ecdsa_signature;   /* secp256k1.h (opaque) */
 typedef struct { unsigned char data[64]; } secp256k1_pubkey;            /* secp256k1.h (opaque) */
+typedef struct { unsigned char data[65]; } secp256k1_ecdsa_recoverable_signature; /* secp256k1_recovery.h (opaque):
+                                                   r, s as 4x64-bit little-endian limbs, recid at data[64] */
 struct pubkey { secp256k1_pubkey pubkey; };                            /* bitcoin/pubkey.h:15-18 */
 struct node_id { u8 k[33]; };                                          /* common/node_id.h:11-13 */
 struct bip340sig { u8 u8[64]; };                                       /* bitcoin/signature.h:145-147 */
@@ -121,6 +123,12 @@ bool check_tx_sig(const struct bitcoin_tx *tx, size_t input_num, const u8 *redee
                   const struct pubkey *key, const struct bitcoin_signature *sig);
 void cln_sigverify_set_tx_hooks(size_t (*script_bytelen)(const void *tal_script),
                                 uint64_t (*input_amount_sat)(const struct bitcoin_tx *tx, size_t input_num));
+
+/* Public-key recovery, batched: ok[i] = secp256k1_ecdsa_recover(secp256k1_ctx, &keys[i].pubkey, &sigs[i], hashes[i].u.u8),
+ * as common/bolt11.c:1043 (invoice without an `n` field) and lightningd/signmessage.c:193 (checkmessage) call it on the
+ * struct secp256k1_ecdsa_recoverable_signature_parse_compact filled.  keys[i] is all zero where ok[i] is false. */
+void ecdsa_recover_batch(const secp256k1_ecdsa_recoverable_signature *sigs, const struct sha256 *hashes, size_t n,
+                         struct pubkey *keys, bool *ok);
 
 /* channeld HTLC loop: ok[i] = check_signed_hash(&hashes[i], &sigs[i].s, key) for one shared key. */
 void check_tx_sigs_batch(const struct sha256_double *hashes, const struct bitcoin_signature *sigs,

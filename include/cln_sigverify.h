@@ -18,6 +18,8 @@
  *                                           channeld/channeld.c:2215-2232)
  *   sv_sha256d_host(...)                    sha256_double()              bitcoin/shadouble.c:7-11
  *   sv_pubkey_parse_host(...)               pubkey_from_der()            bitcoin/pubkey.c:14-24
+ *   sv_recover_host(...)                    secp256k1_ecdsa_recover()    common/bolt11.c:1018-1050,
+ *                                           lightningd/signmessage.c:178-193 (recoverable signatures)
  *   sv_enqueue_* / sv_flush                 the deferral queue a batching caller (gossipd ingest,
  *                                           SURVEY.md §8f N1) sits on; synchronous check_* = enqueue 1 + flush
  *   sv_verify_device(...)                   same kernels on device-resident arrays (bench / multi-GPU)
@@ -175,6 +177,20 @@ typedef struct {
 } sv_tx;
 int sv_verify_tx_host(sv_ctx *ctx, int kind, const sv_tx *txs, const uint8_t *scripts, size_t scripts_len,
                       const uint8_t *key, const uint8_t *sig64, size_t n, uint8_t *verdicts, uint8_t *sighash32_out);
+
+/* ---- ECDSA PUBLIC-KEY RECOVERY, batched: secp256k1_ecdsa_recoverable_signature_parse_compact + secp256k1_ecdsa_recover
+ *      (modules/recovery/main_impl.h:38-57, 137-156) as common/bolt11.c:1018-1050 (invoice signatures without an `n`
+ *      field) and lightningd/signmessage.c:178-193 (checkmessage) call them.  Inputs: msg32[n][32], sig64[n][64] = r_be32 ||
+ *      s_be32 (compact form), recid[n] one byte each.  Outputs per item:
+ *        status[i] = -1  encoding refused: r >= n, s >= n or recid > 3 (never an abort);
+ *        status[i] =  0  no key: r == 0, s == 0, recid & 2 with r >= p - n, x = r (+ n) not on the curve, or Q = infinity;
+ *                        xy64[i] is all zero (as the reference clears its output);
+ *        status[i] =  1  xy64[i] = x_be32 || y_be32 of Q = (-m/r)*G + (s/r)*R, the form sv_pubkey_parse_host writes.
+ *      m = msg mod n is never rejected, and there is no low-S rule: a high s recovers.  Batches of at most small_max items
+ *      take the small-batch kernel, larger ones the throughput kernels in SV_HOST_CHUNK slices; sv_set_profiling events
+ *      cover the scalar-side and curve-side kernels.  Not available in mixed batches or the deferral queue. ---- */
+int sv_recover_host(sv_ctx *ctx, const uint8_t *msg32, const uint8_t *sig64, const uint8_t *recid, size_t n,
+                    uint8_t *xy64, int8_t *status);
 
 /* ---- DEVICE buffers (same SoA layout, device pointers); asynchronous on `stream`
  *      (a cudaStream_t passed as void*; NULL = the context's own stream).  d_verdicts[n] bytes;

@@ -3,6 +3,7 @@
 Everything is built IN-TREE so that the shared objects travel with a gpurun snapshot:
   lightning_b200/libcln_sigverify.so   the product (CUDA kernels + C ABI)            [nvcc]
   tests/host_emul/libemul.so           kernel headers compiled for the host, tests only [g++]
+  tests/host_emul/libemul_recover.so   the same plus the public-key recovery schedules, tests only [g++]
   oracle/libsecp_port.so               the plain-C restatement oracle                 [gcc]
   oracle/_ref/libsecp_ref.so           the unmodified reference, when /root/reference exists [gcc]
 """
@@ -15,6 +16,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 CSRC = os.path.join(ROOT, "lightning_b200", "csrc")
 LIB = os.path.join(ROOT, "lightning_b200", "libcln_sigverify.so")
 EMUL = os.path.join(ROOT, "tests", "host_emul", "libemul.so")
+EMUL_RECOVER = os.path.join(ROOT, "tests", "host_emul", "libemul_recover.so")
 DAEMON = os.path.join(ROOT, "lightning_b200", "cln_sigverifyd")
 
 NVCC_FLAGS = [
@@ -83,16 +85,26 @@ def build_engine(force=False, verbose=False, extra_flags=()):
     return LIB
 
 
-def build_host_emul(force=False):
-    src = os.path.join(ROOT, "tests", "host_emul", "emul.cpp")
-    srcs = _sources(CSRC, (".cuh",)) + [src]
-    if not force and _newer(EMUL, srcs):
-        return EMUL
-    cmd = ["g++", "-O2", "-std=c++17", "-shared", "-fPIC", "-pthread", "-Wall", "-Wno-unused-function", "-o", EMUL, src]
+def _build_emul(out, src, extra_srcs=(), force=False):
+    srcs = _sources(CSRC, (".cuh",)) + [src] + list(extra_srcs)
+    if not force and _newer(out, srcs):
+        return out
+    cmd = ["g++", "-O2", "-std=c++17", "-shared", "-fPIC", "-pthread", "-Wall", "-Wno-unused-function", "-o", out, src]
     r = subprocess.run(cmd, capture_output=True, text=True)
     if r.returncode != 0:
-        raise RuntimeError("g++ (host_emul) failed:\n" + r.stdout + r.stderr)
-    return EMUL
+        raise RuntimeError(f"g++ ({os.path.basename(src)}) failed:\n" + r.stdout + r.stderr)
+    return out
+
+
+def build_host_emul(force=False):
+    d = os.path.join(ROOT, "tests", "host_emul")
+    _build_emul(EMUL_RECOVER, os.path.join(d, "emul_recover.cpp"), [os.path.join(d, "emul.cpp")], force)
+    return _build_emul(EMUL, os.path.join(d, "emul.cpp"), force=force)
+
+
+def build_host_emul_recover(force=False):
+    build_host_emul(force)
+    return EMUL_RECOVER
 
 
 def build_oracle():

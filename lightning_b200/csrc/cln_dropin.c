@@ -214,6 +214,29 @@ bool check_tx_sig(const struct bitcoin_tx *tx, size_t input_num, const u8 *redee
     return v == 1;
 }
 
+void ecdsa_recover_batch(const secp256k1_ecdsa_recoverable_signature *sigs, const struct sha256 *hashes, size_t n,
+                         struct pubkey *keys, bool *ok) {
+    if (n == 0) return;
+    u8 *buf = (u8 *)malloc(n * (32 + 64 + 1 + 64 + 1));
+    if (!buf) die("malloc", -3);
+    u8 *msg = buf, *sig = msg + 32 * n, *recid = sig + 64 * n, *xy = recid + n;
+    int8_t *st = (int8_t *)(xy + 64 * n);
+    for (size_t i = 0; i < n; i++) {
+        memcpy(msg + 32 * i, hashes[i].u.u8, 32);
+        rev32(sig + 64 * i, sigs[i].data);  /* r, s: 4x64-bit little-endian limbs (recovery/main_impl.h:12-35) */
+        rev32(sig + 64 * i + 32, sigs[i].data + 32);
+        recid[i] = sigs[i].data[64];
+    }
+    int rc = sv_recover_host(ctx(), msg, sig, recid, n, xy, st);
+    if (rc != SV_OK) die("sv_recover_host", rc);
+    for (size_t i = 0; i < n; i++) {
+        ok[i] = st[i] == 1;
+        rev32(keys[i].pubkey.data, xy + 64 * i);  /* all zero where nothing was recovered, as the reference leaves it */
+        rev32(keys[i].pubkey.data + 32, xy + 64 * i + 32);
+    }
+    free(buf);
+}
+
 void check_tx_sigs_batch(const struct sha256_double *hashes, const struct bitcoin_signature *sigs,
                          const struct pubkey *key, size_t n, bool *ok) {
     if (n == 0) return;

@@ -11,6 +11,7 @@
 //       k_final_ecdsa33, k_final_schnorr_ns   batched division that settles the parked linear conditions of kinds 3 / 4
 //       k_final_schnorr                  plain BIP-340 flow: affine R from the parked Jacobian R (batched inversion)
 //       k_small<kind>                    one-launch latency path for small batches (5 warps per 32 verifications)
+//       k_prep_recover_*, k_main<5>, k_final_recover, k_small<5>   public-key recovery (sv_recover_host)
 //       k_main_shared, k_dedup_*, k_sharedkey_build_many   one multiples table per distinct key (same-key / gossip batches)
 //       k_gossip_slice / _status, k_bip143, k_mixed_*       callers' data formats on the device (rows N1, N2, C3)
 //       k_sb_* (batch.cu)                BIP-340 batch verification by random linear combination
@@ -125,6 +126,54 @@ __global__ void __launch_bounds__(128) k_prep_finish(const u8* msg, const u8* si
     work[i] = w;
 }
 
+// scalar side of public-key recovery, split as for ECDSA: here r is the scalar to invert (recid in a byte array of its own)
+__global__ void __launch_bounds__(64) k_prep_recover_inv(const u8* msg, const u8* sig, const u8* recid, size_t n, sv_work* work) {
+    size_t t = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    size_t base = t * SV_PREP_BATCH;
+    if (base >= n) return;
+    int cnt = (int)((n - base < SV_PREP_BATCH) ? (n - base) : SV_PREP_BATCH);
+    sc rv[SV_PREP_BATCH];
+    u32 okmask = 0, parsedmask = 0;
+#pragma unroll 1
+    for (int j = 0; j < SV_PREP_BATCH; j++) {
+        sc r, s, m;
+        bool ok = false, parsed = false;
+        if (j < cnt) recover_parse(r, s, m, ok, parsed, sig + 64 * (base + j), msg + 32 * (base + j), recid[base + j]);
+        parsedmask |= (parsed ? 1u : 0u) << j;
+        if (!ok) {
+#pragma unroll
+            for (int k = 0; k < 8; k++) r.v[k] = (k == 0);
+        }
+        okmask |= (ok ? 1u : 0u) << j;
+        rv[j] = r;
+    }
+    sc_batch_inverse(rv, SV_PREP_BATCH);
+#pragma unroll 1
+    for (int j = 0; j < cnt; j++) {
+        u32* w = reinterpret_cast<u32*>(work + base + j);
+        fe_to_words(w, *reinterpret_cast<const fe*>(&rv[j]));  // words 0..7: r^-1
+        w[8] = ((okmask >> j) & 1u) | (((parsedmask >> j) & 1u) << 1);
+    }
+}
+__global__ void __launch_bounds__(128) k_prep_recover_finish(const u8* msg, const u8* sig, const u8* recid, size_t n,
+                                                             sv_work* work) {
+    size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const u32* wi = reinterpret_cast<const u32*>(work + i);
+    sc rinv;
+    fe tmp;
+    fe_from_words(tmp, wi);
+#pragma unroll
+    for (int k = 0; k < 8; k++) rinv.v[k] = tmp.v[k];
+    u32 f = wi[8];
+    sc r, s, m;
+    bool ok, parsed;
+    recover_parse(r, s, m, ok, parsed, sig + 64 * i, msg + 32 * i, recid[i]);
+    sv_work w;
+    recover_finish_prep(w, (f & 1u) != 0, (f & 2u) != 0, r, s, m, rinv);
+    work[i] = w;
+}
+
 __global__ void __launch_bounds__(128) k_prep_schnorr(const u8* msg, const u8* key, const u8* sig, size_t n,
                                                       sv_work* work) {
     size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -153,7 +202,8 @@ template <int KIND>
 __global__ void __launch_bounds__(SV_MAIN_BLOCK, SV_MAIN_MINB)
     k_main(sv_work* work, const u8* __restrict__ key, const u8* __restrict__ sig, size_t n,
            const ge_mem* __restrict__ gtab, qtab_entry* scratch, u8* __restrict__ verdict, u8* keyok) {
-    const size_t keylen = (KIND == SV_KIND_ECDSA33 || KIND == SV_KIND_ECDSA33_NS) ? 33 : (KIND == SV_KIND_ECDSA_XY ? 64 : 32);
+    const size_t keylen = (KIND == SV_KIND_ECDSA33 || KIND == SV_KIND_ECDSA33_NS) ? 33
+                          : (KIND == SV_KIND_ECDSA_XY ? 64 : (KIND == SV_KIND_RECOVER ? 1 : 32));
 #ifdef SV_COMB_SMEM
     // VARIANT: the 17 x 128-entry 8-bit comb (136 KiB) is staged in shared memory once per (persistent) CTA by ONE bulk
     // asynchronous copy (cp.async.bulk: the TMA engine, UBLKCP in SASS), completion signalled on an mbarrier
@@ -226,6 +276,16 @@ __global__ void __launch_bounds__(SV_MAIN_BLOCK, SV_MAIN_MINB)
             gej R;
             ecmult_uniform(R, w, Q, gtab, tab, part);
             if (active) schnorr_park(reinterpret_cast<sv_jac*>(work + i), R, ok);
+        } else if (KIND == SV_KIND_RECOVER) {
+            // public-key recovery: the recid byte sits in the key slot; Q is parked in the work record and
+            // k_final_recover turns it into an affine key (batched inversion)
+            const u32 recid = key[j];
+            const u32 flags = w->flags;
+            ge R;
+            bool ok = recover_lift(R, sig + 64 * j, recid) && recover_lift_allowed(flags, recid);
+            gej Q;
+            ecmult_uniform(Q, w, R, gtab, tab, part);
+            if (active) recover_park(reinterpret_cast<sv_jac*>(work + i), Q, ok, (flags & SV_WF_PARSED) != 0);
         } else {
             bool kd;
             u32 v = verify_curve_side(KIND, w, key + keylen * j, sig + 64 * j, gtab, tab, &kd, part);
@@ -245,7 +305,8 @@ template <int KIND, bool NOSQRT>
 __global__ void __launch_bounds__(160, 1)
     k_small(const u8* __restrict__ msg, const u8* __restrict__ key, const u8* __restrict__ sig, size_t n,
             const ge_mem* __restrict__ gtab, u8* __restrict__ verdict, u8* __restrict__ aux) {
-    constexpr int keylen = (KIND == SV_KIND_ECDSA33) ? 33 : (KIND == SV_KIND_ECDSA_XY ? 64 : 32);
+    // SV_KIND_RECOVER: the key slot holds the recid byte, verdict receives the status bytes and aux the 64-byte keys
+    constexpr int keylen = (KIND == SV_KIND_ECDSA33) ? 33 : (KIND == SV_KIND_ECDSA_XY ? 64 : (KIND == SV_KIND_RECOVER ? 1 : 32));
     __shared__ sv_small_item items[SV_SMALL_ITEMS];
     __shared__ __align__(16) u8 in_msg[SV_SMALL_ITEMS * 32];
     __shared__ __align__(16) u8 in_key[SV_SMALL_ITEMS * 64];
@@ -264,9 +325,14 @@ __global__ void __launch_bounds__(160, 1)
     const u8* m = in_msg + 32 * j;
     const u8* k = in_key + keylen * j;
     const u8* sg = in_sig + 64 * j;
-    if (warp == 0) {
-        if (NOSQRT) small_key_side_ns(KIND, k, it); else small_key_side(KIND, k, it);
-    } else if (warp == 1) small_scalar_side(KIND, m, k, sg, it);
+    if constexpr (KIND == SV_KIND_RECOVER) {
+        if (warp == 0) small_recover_key_side(sg, k[0], it);   // lift R and tabulate it
+        else if (warp == 1) small_recover_scalar_side(m, sg, k[0], it);
+    } else {
+        if (warp == 0) {
+            if (NOSQRT) small_key_side_ns(KIND, k, it); else small_key_side(KIND, k, it);
+        } else if (warp == 1) small_scalar_side(KIND, m, k, sg, it);
+    }
     __syncthreads();
     // phase B: warps 0..3 run the half ladders on lane PAIRS (warp w: half w >> 1, items 16 (w & 1) + lane / 2), warp 4 the comb
     if (warp < 4) {
@@ -277,7 +343,9 @@ __global__ void __launch_bounds__(160, 1)
         small_comb(it, gtab);
     }
     __syncthreads();
-    if (warp == 0) {
+    if constexpr (KIND == SV_KIND_RECOVER) {
+        if (warp == 0 && active) small_recover_finish(it, k[0], aux + 64 * (base + lane), verdict + base + lane);
+    } else if (warp == 0) {
         bool kd = false;
         u32 v = NOSQRT ? small_finish_ns(KIND, it, k, sg, gtab, aux ? &kd : nullptr) : small_finish(KIND, it, sg, &kd);
         if (active) {
@@ -507,6 +575,15 @@ __global__ void __launch_bounds__(64) k_final_schnorr(const sv_work* work, const
     if (base >= n) return;
     int cnt = (int)((n - base < SV_FINAL_BATCH) ? (n - base) : SV_FINAL_BATCH);
     schnorr_final_batch(verdict + base, reinterpret_cast<const sv_jac*>(work) + base, sig + 64 * base, cnt);
+}
+
+// public-key recovery: affine keys from the parked Q (batched inversion), status 1 / 0 / -1 as a byte
+__global__ void __launch_bounds__(64) k_final_recover(const sv_work* work, size_t n, u8* xy64, u8* status) {
+    size_t t = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    size_t base = t * SV_FINAL_BATCH;
+    if (base >= n) return;
+    int cnt = (int)((n - base < SV_FINAL_BATCH) ? (n - base) : SV_FINAL_BATCH);
+    recover_final_batch(xy64 + 64 * base, status + base, reinterpret_cast<const sv_jac*>(work) + base, cnt);
 }
 
 static_assert(sizeof(sv_ns_park) == sizeof(sv_work), "D, B, c are parked in place of the work record");
@@ -1771,6 +1848,103 @@ extern "C" int sv_verify_mixed_host(sv_ctx* ctx, const uint8_t* kinds, const uin
     if (rc) return rc;
     CK(cudaMemcpyAsync(verdicts, d_o, n, cudaMemcpyDeviceToHost, st));
     CK(cudaStreamSynchronize(st));
+    return SV_OK;
+}
+
+// ---- public-key recovery (secp256k1_ecdsa_recover; verify.cuh "public-key recovery") -----------------------------------
+// inputs on the device: recid[n] bytes, keys to d_xy (64 bytes per item), status bytes (int8_t) to d_status
+static int launch_recover(sv_ctx* ctx, const u8* d_msg, const u8* d_recid, const u8* d_sig, size_t n, u8* d_xy, u8* d_status,
+                          cudaStream_t st) {
+    if (n == 0) return SV_OK;
+    if (n <= ctx->small_max) {
+        unsigned grid = (unsigned)((n + SV_SMALL_ITEMS - 1) / SV_SMALL_ITEMS);
+        if (ctx->profiling) cudaEventRecord(ctx->ev[0], st);
+        if (ctx->profiling) cudaEventRecord(ctx->ev[1], st);
+        k_small<SV_KIND_RECOVER, false><<<grid, 160, 0, st>>>(d_msg, d_recid, d_sig, n, ctx->d_gtab, d_status, d_xy);
+        if (ctx->profiling) cudaEventRecord(ctx->ev[2], st);
+        ctx->launches += 1;
+        CK(cudaGetLastError());
+        return SV_OK;
+    }
+    sv_ctx::slot_t* sl = nullptr;
+    int rc = acquire_slot(ctx, n, st, &sl);
+    if (rc) return rc;
+    apply_l2_policy(ctx, st, sl->d_scratch);
+    sv_work* work = sl->d_work;
+    if (ctx->profiling) cudaEventRecord(ctx->ev[0], st);
+    size_t threads = (n + SV_PREP_BATCH - 1) / SV_PREP_BATCH;
+    k_prep_recover_inv<<<(unsigned)((threads + 63) / 64), 64, 0, st>>>(d_msg, d_sig, d_recid, n, work);
+    k_prep_recover_finish<<<(unsigned)((n + 127) / 128), 128, 0, st>>>(d_msg, d_sig, d_recid, n, work);
+    if (ctx->profiling) cudaEventRecord(ctx->ev[1], st);
+    size_t want = (n + SV_MAIN_BLOCK - 1) / SV_MAIN_BLOCK;
+    unsigned grid = (unsigned)(want < (size_t)ctx->main_grid ? want : (size_t)ctx->main_grid);
+    k_main<SV_KIND_RECOVER><<<grid, SV_MAIN_BLOCK, SV_MAIN_SMEM, st>>>(work, d_recid, d_sig, n, ctx->d_gtab, sl->d_scratch, nullptr, nullptr);
+    threads = (n + SV_FINAL_BATCH - 1) / SV_FINAL_BATCH;
+    k_final_recover<<<(unsigned)((threads + 63) / 64), 64, 0, st>>>(work, n, d_xy, d_status);
+    if (ctx->profiling) cudaEventRecord(ctx->ev[2], st);
+    ctx->launches += 4;
+    CK(cudaGetLastError());
+    return release_slot(ctx, sl, st);
+}
+
+extern "C" int sv_recover_host(sv_ctx* ctx, const uint8_t* msg32, const uint8_t* sig64, const uint8_t* recid, size_t n,
+                               uint8_t* xy64, int8_t* status) {
+    if (!ctx || (n && (!msg32 || !sig64 || !recid || !xy64 || !status))) return SV_ERR_ARG;
+    if (n == 0) return SV_OK;
+    dev_guard dg__;
+    CK(dg__.enter(ctx->device));
+    if (n <= ctx->small_max) {
+        // pinned staging block as in sv_verify_host: recids in the second byte per item of the verdict area, keys come
+        // back through the key area (the kernel never reads it for this kind)
+        const size_t cap = ctx->small_cap;
+        u8 *hm = ctx->h_small, *hk = hm + 32 * cap, *hs = hk + 64 * cap, *hv = hs + 64 * cap;
+        memcpy(hm, msg32, 32 * n);
+        memcpy(hv + cap, recid, n);
+        memcpy(hs, sig64, 64 * n);
+        int rc = launch_recover(ctx, hm, hv + cap, hs, n, hk, hv, ctx->stream);
+        if (rc) return rc;
+        CK(cudaStreamSynchronize(ctx->stream));
+        memcpy(xy64, hk, 64 * n);
+        memcpy(status, hv, n);
+        return SV_OK;
+    }
+    size_t chunk = n < SV_HOST_CHUNK ? n : SV_HOST_CHUNK;
+    int rc = ensure_staging(ctx, chunk);
+    if (rc) return rc;
+    rc = ensure_gbuf(ctx, 64 * chunk);  // the keys of one chunk
+    if (rc) return rc;
+    u8* d_xy = ctx->g_buf;
+    // the slicing and stream pipeline of sv_verify_host; the recid bytes travel in the key staging array
+    const size_t wave = (size_t)ctx->main_grid * SV_MAIN_BLOCK;
+    for (size_t off = 0; off < n; off += chunk) {
+        size_t c = (n - off < chunk) ? (n - off) : chunk;
+        size_t done = 0;
+        int k = 0;
+        const bool piped = c > 2 * wave;
+        while (done < c) {
+            size_t want = (k == 0) ? wave + c % wave : 6 * wave;
+            size_t s = (c - done <= want + 2 * wave) ? (c - done) : want;
+            if (k >= 7) s = c - done;
+            cudaStream_t cs = piped ? ctx->copy_stream : ctx->stream;
+            cudaStream_t ks = (piped && (k & 1)) ? ctx->stream2 : ctx->stream;
+            CK(cudaMemcpyAsync(ctx->d_msg + 32 * done, msg32 + 32 * (off + done), 32 * s, cudaMemcpyHostToDevice, cs));
+            CK(cudaMemcpyAsync(ctx->d_key + done, recid + off + done, s, cudaMemcpyHostToDevice, cs));
+            CK(cudaMemcpyAsync(ctx->d_sig + 64 * done, sig64 + 64 * (off + done), 64 * s, cudaMemcpyHostToDevice, cs));
+            if (cs != ks) {
+                CK(cudaEventRecord(ctx->h2d_ev[k], cs));
+                CK(cudaStreamWaitEvent(ks, ctx->h2d_ev[k], 0));
+            }
+            rc = launch_recover(ctx, ctx->d_msg + 32 * done, ctx->d_key + done, ctx->d_sig + 64 * done, s, d_xy + 64 * done,
+                                ctx->d_verdict + done, ks);
+            if (rc) return rc;
+            CK(cudaMemcpyAsync(xy64 + 64 * (off + done), d_xy + 64 * done, 64 * s, cudaMemcpyDeviceToHost, ks));
+            CK(cudaMemcpyAsync(status + off + done, ctx->d_verdict + done, s, cudaMemcpyDeviceToHost, ks));
+            done += s;
+            k++;
+        }
+        CK(cudaStreamSynchronize(ctx->stream));
+        if (piped) CK(cudaStreamSynchronize(ctx->stream2));
+    }
     return SV_OK;
 }
 

@@ -32,6 +32,7 @@
 #define SV_KIND_SCHNORR 2   // msg32 | xonly32            | sig64 (R.x||s)    BIP-340
 #define SV_KIND_ECDSA33_NS 3  // internal: kind 0 through the flow that never takes the square root (see below)
 #define SV_KIND_SCHNORR_NS 4  // internal: kind 2 likewise
+#define SV_KIND_RECOVER 5     // internal: msg32 | recid (1 byte in the key slot) | sig64 (r||s) -> public key (see "recovery")
 
 // G comb table geometry: rows 0..14 hold d*B_i for d = 1..32768, row 15 holds d = 1..65536
 #define SV_GT_ROW 32768
@@ -524,6 +525,116 @@ SV_HD void schnorr_final_batch(u8* verdict, const sv_jac* jac, const u8* sig64, 
         fe_set_b32(rx, sig64 + 64 * i);
         bool good = usable && !fe_is_odd(a.y) && fe_equal(rx, a.x);  // main_impl.h:255-264
         verdict[i] = good ? 1 : 0;
+    }
+}
+
+// ---- public-key recovery (secp256k1_ecdsa_recover, modules/recovery/main_impl.h:87-156) --------------------------------
+// Q = (-m/r)*G + (s/r)*R with R = lift(r (+ n if recid & 2)), y(R) odd iff recid & 1.  The same split as a verification:
+// the scalar side writes u1 = -m/r into the comb digits and u2 = s/r into the GLV halves, the curve side lifts R (one
+// square root), runs the same double-scalar multiplication and parks Q; the affine key needs one field inversion, batched
+// 16 at a time like the BIP-340 final step.  Outcomes per item:
+//   -1  encoding refused: r >= n, s >= n (recoverable_signature_parse_compact, main_impl.h:38-57) or recid > 3
+//    0  recovery failed, key all zero: r == 0, s == 0, recid & 2 with r >= p - n, no curve point with x = r (+ n), Q = inf
+//    1  key = affine x || y of Q, big-endian.  No low-S rule: a high s recovers.
+#define SV_RECOVER_REFUSED 0xFFu  // the status byte of outcome -1 (int8_t -1)
+
+// scalar side of one item, given 1/r (r != 0) or anything (invalid item).  ok: r, s in range and non-zero, recid <= 3.
+SV_HD void recover_parse(sc& r, sc& s, sc& m, bool& ok, bool& parsed, const u8* sig64, const u8* msg32, u32 recid) {
+    bool ovr, ovs;
+    sc_set_b32(r, sig64, &ovr);
+    sc_set_b32(s, sig64 + 32, &ovs);
+    sc_set_b32(m, msg32, nullptr);  // m mod n, never rejected (main_impl.h:138)
+    parsed = !ovr && !ovs && recid <= 3u;
+    ok = parsed && !sc_is_zero(r) && !sc_is_zero(s);  // ecdsa_sig_recover, main_impl.h:93-95
+}
+SV_HD void recover_finish_prep(sv_work& w, bool ok, bool parsed, const sc& r, const sc& s, const sc& m, const sc& rinv) {
+    if (!ok) {
+        work_set_invalid(w);
+        w.flags = parsed ? SV_WF_PARSED : 0u;
+        return;
+    }
+    sc u1, u2;
+    sc_mul(u1, rinv, m);
+    sc_negate(u1, u1);  // -m/r  (main_impl.h:113-114)
+    sc_mul(u2, rinv, s);  // s/r (:115)
+    SV_UNROLL
+    for (int i = 0; i < 5; i++) w.pad[i] = 0;
+    sc_prepare_u2(w, u2);
+#ifdef SV_COMB_SMEM
+    sc_prepare_u1_smem(w, u1);
+#else
+    sc_prepare_u1(w, u1);
+#endif
+    const u32 pmn[8] = {0x2FC9BAEEu, 0x402DA172u, 0x50B75FC4u, 0x45512319u, 0x00000001u, 0, 0, 0};  // p - n
+    u32 t[8];
+    u32 bw = u256_sub(t, r.v, pmn);
+    w.flags = SV_WF_VALID | SV_WF_PARSED | (bw ? SV_WF_R_PLUS_N : 0u);
+}
+
+// R from r and the recovery id, without the range check of r + n (the scalar side's SV_WF_R_PLUS_N, which the caller
+// ANDs in): false if x^3 + 7 is not a square (main_impl.h:97-107).  No early exit: see key_decode.
+SV_HD bool recover_lift(ge& R, const u8* sig64, u32 recid) {
+    fe x;
+    fe_set_b32(x, sig64);  // r < n < p for every item that can succeed
+    if (recid & 2u) {
+        fe nn;
+        SV_UNROLL
+        for (int i = 0; i < 8; i++) nn.v[i] = SC_N[i];
+        u256_add(x.v, x.v, nn.v);  // r + n < p when it counts
+    }
+    return ge_set_xo(R, x, (recid & 1u) != 0);
+}
+SV_HD bool recover_lift_allowed(u32 flags, u32 recid) {
+    return (flags & SV_WF_VALID) != 0 && (!(recid & 2u) || (flags & SV_WF_R_PLUS_N) != 0);
+}
+
+// Q parked in place of the work record: ok = a point may come out, pad[0] = the encoding parsed (status 0 rather than -1)
+SV_HD void recover_park(sv_jac* out, const gej& Q, bool ok, bool parsed) {
+    schnorr_park(out, Q, ok);
+    out->pad[0] = parsed ? 1u : 0u;
+}
+
+SV_HD void recover_emit(u8* xy64, u8* status, const ge* a, bool parsed) {
+    if (a) {
+        fe_get_b32(xy64, a->x);
+        fe_get_b32(xy64 + 32, a->y);
+        *status = 1;
+    } else {
+        for (int k = 0; k < 64; k++) xy64[k] = 0;  // main_impl.h:150-156
+        *status = parsed ? 0u : SV_RECOVER_REFUSED;
+    }
+}
+
+// keys and statuses for cnt (<= SV_FINAL_BATCH) consecutive parked results: one Fermat inversion for all their Z's
+SV_HD void recover_final_batch(u8* xy64, u8* status, const sv_jac* jac, int cnt) {
+    fe pre[SV_FINAL_BATCH];
+    fe acc, one;
+    fe_set_u32(one, 1);
+    for (int i = 0; i < cnt; i++) {
+        fe z;
+        fe_from_words(z, jac[i].z);
+        bool usable = jac[i].ok && !jac[i].inf && !fe_is_zero(z);
+        if (!usable) z = one;
+        if (i == 0) pre[0] = z; else fe_mul(pre[i], pre[i - 1], z);
+    }
+    fe_inv(acc, pre[cnt - 1]);
+    for (int i = cnt - 1; i >= 0; i--) {
+        fe z, zi;
+        fe_from_words(z, jac[i].z);
+        bool usable = jac[i].ok && !jac[i].inf && !fe_is_zero(z);
+        if (!usable) z = one;
+        if (i > 0) {
+            fe_mul(zi, acc, pre[i - 1]);
+            fe_mul(acc, acc, z);
+        } else {
+            zi = acc;
+        }
+        gej Q;
+        fe_from_words(Q.x, jac[i].x);
+        fe_from_words(Q.y, jac[i].y);
+        ge a;
+        ge_set_gej_zinv(a, Q, zi);
+        recover_emit(xy64 + 64 * i, status + i, usable ? &a : nullptr, jac[i].pad[0] != 0);
     }
 }
 
@@ -1270,6 +1381,49 @@ SV_HD void small_half_ladder_pair(const pair_lane& L, sv_small_item* it, int hal
     gej R;
     ecmult_half_ladder_pair(L, R, half ? it->w.k2 : it->w.k1, half != 0, it->tab);
     if (L.role == 0) small_jac_store(half ? &it->r2 : &it->r1, R);
+}
+
+// ---- recovery on the small-batch path: warp 0 lifts R and builds its table in place of the key side, warp 1 runs the
+// scalar side with a lone inversion of r, the half ladders and the comb are unchanged, and the finish leaves Jacobian
+// coordinates with one field inversion per item (no batch to share it with here)
+SV_HD void small_recover_key_side(const u8* sig64, u32 recid, sv_small_item* it) {
+    ge R;
+    it->key_ok = recover_lift(R, sig64, recid) ? 1u : 0u;
+    fe zc;
+    qtable_build(it->tab, zc, R);
+    fe_to_words(it->zc, zc);
+}
+SV_HD void small_recover_scalar_side(const u8* msg32, const u8* sig64, u32 recid, sv_small_item* it) {
+    sc r, s, m, rinv, d;
+    bool ok, parsed;
+    recover_parse(r, s, m, ok, parsed, sig64, msg32, recid);
+    d = r;
+    if (!ok) {
+        SV_UNROLL
+        for (int k = 0; k < 8; k++) d.v[k] = (k == 0);
+    }
+    sc_inverse_var(rinv, d);
+    recover_finish_prep(it->w, ok, parsed, r, s, m, rinv);
+}
+SV_HD void small_recover_finish(sv_small_item* it, u32 recid, u8* xy64, u8* status) {
+    gej R, T;
+    small_jac_load(R, &it->r1);
+    small_jac_load(T, &it->r2);
+    gej_add_gej(R, R, T);  // on the scaled curve
+    fe zc;
+    fe_from_words(zc, it->zc);
+    fe_mul(R.z, R.z, zc);
+    small_jac_load(T, &it->p3);
+    gej_add_gej(R, R, T);
+    const u32 flags = it->w.flags;
+    const bool usable = recover_lift_allowed(flags, recid) && it->key_ok != 0 && !R.inf;
+    ge a;
+    if (usable) {
+        fe zi;
+        fe_inv_var(zi, R.z);
+        ge_set_gej_zinv(a, R, zi);
+    }
+    recover_emit(xy64, status, usable ? &a : nullptr, (flags & SV_WF_PARSED) != 0);
 }
 
 // the three phases run one after another (host build of the kernel source, tests/host_emul)

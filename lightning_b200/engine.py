@@ -73,6 +73,7 @@ def load_library():
     lib.sv_flush.argtypes = [vp, vp, sz]
     lib.sv_sha256d_host.argtypes = [vp, vp, sz, vp, vp, sz, vp]
     lib.sv_pubkey_parse_host.argtypes = [vp, vp, sz, vp, vp]
+    lib.sv_recover_host.argtypes = [vp, vp, vp, vp, sz, vp, vp]
     lib.sv_synth_device.argtypes = [vp, i, ctypes.c_uint64, sz, vp, vp, vp, vp]
     lib.sv_selftest_host.argtypes = [vp, i, vp, vp, sz, vp]
     lib.sv_verify_mixed_host.argtypes = [vp, vp, vp, vp, vp, sz, vp]
@@ -232,6 +233,21 @@ class SigVerifier:
         self._check(self.lib.sv_pubkey_parse_host(self._ctx, key33.ctypes.data, n, xy.ctypes.data, ok.ctypes.data),
                     "sv_pubkey_parse_host")
         return xy, ok
+
+    def recover(self, msg32, sig64, recid):
+        """secp256k1_ecdsa_recover, batched (common/bolt11.c:1018-1050, lightningd/signmessage.c:178-193).  msg32 (n, 32),
+        sig64 (n, 64) compact r || s, recid (n,) bytes.  Returns (xy64 (n, 64) uint8, status (n,) int8): 1 = key x || y,
+        0 = no key (all zero), -1 = encoding refused (r >= n, s >= n or recid > 3)."""
+        msg32, sig64 = _u8(msg32, 32), _u8(sig64, 64)
+        recid = np.ascontiguousarray(recid, dtype=np.uint8).reshape(-1)
+        n = msg32.shape[0]
+        if sig64.shape[0] != n or recid.shape[0] != n:
+            raise ValueError("length mismatch")
+        xy = np.zeros((n, 64), dtype=np.uint8)
+        status = np.zeros(n, dtype=np.int8)
+        self._check(self.lib.sv_recover_host(self._ctx, msg32.ctypes.data, sig64.ctypes.data, recid.ctypes.data, n,
+                                             xy.ctypes.data, status.ctypes.data), "sv_recover_host")
+        return xy, status
 
     def verify_mixed(self, kinds, msg32, key64, sig64):
         """Interleaved batch: kinds (n,) uint8 SV_KIND_* tags, keys in 64-byte slots; verdicts in item order."""
